@@ -70,7 +70,33 @@ def parse():
                    help="K3 sweep: cp.async.bulk (TMA) pipeline or the per-thread-load kernel (A/B; sets GG_ADAM_PATH)")
     p.add_argument("--phase", default="sample", choices=["sample", "reward", "adam", "bfs", "update"],
                    help="what to time: the D-sampling pass (the BASELINE metric) or one of the other kernels of the path")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the (center, neighbor, label) rows of the last timed D-sampling step as DIR/<name>.npy "
+                        "(float64; a fixed sample of %d rows when there are more), to compare two builds output for output"
+                        % DUMP_ROWS)
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.phase != "sample"):
+        p.error("--dump-outputs writes the D-sampling pass of --impl b200 --phase sample")
+    return args
+
+
+DUMP_ROWS = 1 << 20      # 4 float64 arrays of this many rows: 32 MiB, half of the 64 MB a dump may take
+
+
+def dump_rows(dirname, out):
+    """The rows prepare_data_for_d returns (graph_gan.py:192-201) as the last step of `out` left them in its plan's
+    buffers, plus row_index.npy (which rows: all of them, or a fixed seeded sample) and n_rows.npy."""
+    p = out.plan
+    n = int(p.n_rows.item())
+    idx = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {"n_rows": np.array([n]), "row_index": idx}
+    for name, rows in zip(("center", "neighbor", "label"), p.rows):
+        arrays[name] = rows[:n].cpu().numpy()[idx]
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a.astype(np.float64))
 
 
 def make_inputs(args, rank):
@@ -535,6 +561,8 @@ def run_b200(args):
     clocks.wait_first()
     ms, cnts, t_start, t_end, last_out = timed(False)
     clk = clocks.stop(t_start, t_end)
+    if rank == 0 and args.dump_outputs:         # before the e2e passes below overwrite the plan's row buffers
+        dump_rows(args.dump_outputs, last_out)
     parity = None
     if rank == 0 and args.verify > 0:
         parity = _verify(args, hg, emb_h, roots, trees, last_out, smp, dev, args.seed, 2000 + args.steps - 1)

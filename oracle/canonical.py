@@ -5,6 +5,7 @@ The walk follows src/GraphGAN/graph_gan.py:182-270 with the arithmetic pinned do
 CUDA kernels can be compared bit-for-bit.  Never imported by graphgan_b200/.
 """
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -17,11 +18,28 @@ NOTRUN, DONE, VOID, SKIPPED = 0, 1, 2, 3
 RNG_PHILOX, RNG_STREAM = 0, 1
 
 
+def _source_hash():
+    h = hashlib.sha256()
+    for f in ("gg_oracle.c", "gg_oracle.h", "Makefile"):
+        h.update(f.encode())
+        with open(os.path.join(HERE, f), "rb") as src:
+            h.update(src.read())
+    return h.hexdigest()
+
+
 def build(force=False):
+    """Rebuild libgg_oracle.so when it is missing or was built from other sources.  The sources' content hash is
+    kept in a sidecar file, not their mtimes: a copied tree has new mtimes, and may be read-only."""
     so = os.path.join(HERE, "libgg_oracle.so")
-    src = [os.path.join(HERE, f) for f in ("gg_oracle.c", "gg_oracle.h", "Makefile")]
-    if force or not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in src):
-        subprocess.check_call(["make", "-C", HERE, "-s", "-B", "libgg_oracle.so"])
+    stamp = so + ".hash"
+    want = _source_hash()
+    if not force and os.path.exists(so) and os.path.exists(stamp):
+        with open(stamp) as f:
+            if f.read().strip() == want:
+                return so
+    subprocess.check_call(["make", "-C", HERE, "-s", "-B", "libgg_oracle.so"])
+    with open(stamp, "w") as f:
+        f.write(want + "\n")
     return so
 
 

@@ -30,9 +30,11 @@ def load(name):
     c = Case({k: z[k] for k in z.files})
     n, d, seed = int(c["n_node"]), int(c["d"]), int(c["seed"])
     rs = np.random.RandomState(seed + 1000)
-    if "pretrain_q1e6" in c:
+    if "pretrain_q1e6_bytes" in c:
+        b = c["pretrain_q1e6_bytes"].astype(np.int64)          # byte planes of pretrain_q1e6 + 2**23
+        q = (b[0] | b[1] << 8 | b[2] << 16) - (1 << 23)
         fill = np.random.RandomState(int(c["pretrain_fill_seed"])).rand(n, d)
-        fill[c["pretrain_ids"]] = c["pretrain_q1e6"].astype(np.float64) / 1e6
+        fill[c["pretrain_ids"]] = q.astype(np.float64) / 1e6
         emb_g, emb_d = fill, fill.copy()
     else:
         emb_g = rs.normal(0, 0.5, size=(n, d))

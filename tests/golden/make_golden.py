@@ -1,15 +1,15 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in tests/golden/ by running the UNMODIFIED reference.
 
-Run in the authoring container only (needs /root/reference; the GPU box has no copy):
+Needs a checkout of the reference (hwwang55/GraphGAN); the tests only read the fixtures:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 What runs: the reference's own host half -- ``GraphGAN.construct_trees``, ``sample``,
 ``prepare_data_for_d``, ``prepare_data_for_g``, ``get_node_pairs_from_path``
-(/root/reference/src/GraphGAN/graph_gan.py:84-108, 182-291) and ``utils.read_edges`` /
-``utils.softmax`` (/root/reference/src/utils.py:12-47, 131-133) -- imported from
-/root/reference, never copied.  TensorFlow 1.8 is not installable here, so a stub
+(src/GraphGAN/graph_gan.py:84-108, 182-291) and ``utils.read_edges`` /
+``utils.softmax`` (src/utils.py:12-47, 131-133) -- imported from the
+reference checkout, never copied.  TensorFlow 1.8 is not installed, so a stub
 ``tensorflow`` module satisfies the import and a stub session answers the two fetches the
 sampling code makes (``generator.all_score`` = fp32 E.E^T + b, generator.py:21;
 ``discriminator.reward`` = log(1+exp(clip(score,-10,10))), discriminator.py:21-24,33-34)
@@ -27,7 +27,7 @@ import types
 
 import numpy as np
 
-REF = "/root/reference"
+REF = None  # the reference checkout, set by main() from the command line
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -122,12 +122,14 @@ class Recorder:
         np.random.choice = self._choice
         np.random.rand = self._rand
 
-    def arrays(self, prefix):
+    def arrays(self, prefix, steps=None):
+        """The trace; ``steps`` keeps only the first steps (the per-root draws stay complete)."""
+        k = len(self.chosen) if steps is None else min(steps, len(self.chosen))
         return {
-            prefix + "step_draw": np.asarray(self.step_draw, np.int64),
-            prefix + "cand_flat": np.asarray(self.cand_flat, np.int32),
-            prefix + "cand_ptr": np.asarray(self.cand_ptr, np.int64),
-            prefix + "chosen": np.asarray(self.chosen, np.int32),
+            prefix + "step_draw": np.asarray(self.step_draw[:k], np.int64),
+            prefix + "cand_flat": np.asarray(self.cand_flat[:self.cand_ptr[k]], np.int32),
+            prefix + "cand_ptr": np.asarray(self.cand_ptr[:k + 1], np.int64),
+            prefix + "chosen": np.asarray(self.chosen[:k], np.int32),
             prefix + "root_draw": np.asarray(self.root_draw, np.int64),
         }
 
@@ -174,7 +176,7 @@ def sha(*arrs):
 
 
 def run_case(gg_mod, ref_utils, name, train_edges, test_edges, d, seed, emb=None, trace_g=True,
-             keep_parent=True, n_sample_gen=None, extra=None):
+             keep_parent=True, n_sample_gen=None, extra=None, d_trace_steps=None):
     import config as ref_config  # the reference's config module
     tmp = tempfile.mkdtemp()
     trf, tef = os.path.join(tmp, "train.txt"), os.path.join(tmp, "test.txt")
@@ -249,6 +251,7 @@ def run_case(gg_mod, ref_utils, name, train_edges, test_edges, d, seed, emb=None
         "d_center": np.asarray(center, np.int32), "d_neighbor": np.asarray(neighbor, np.int32),
         "d_labels": np.asarray(labels, np.int32),
         "d_draws": np.int64(rec_d.draws), "total_draws": np.int64(total_draws),
+        "d_steps": np.int64(len(rec_d.chosen)), "d_sum_l": np.int64(rec_d.cand_ptr[-1]),
         "mutated": np.asarray(mutated, np.int32).reshape(-1, 2),
         "g_n_pairs": np.int64(len(node_1)),
         "g_pairs_sha": np.frombuffer(bytes.fromhex(sha(np.asarray(node_1, np.int32), np.asarray(node_2, np.int32))),
@@ -260,7 +263,7 @@ def run_case(gg_mod, ref_utils, name, train_edges, test_edges, d, seed, emb=None
     }
     if keep_parent:
         out["parent"] = parent0
-    out.update(rec_d.arrays("dtr_"))
+    out.update(rec_d.arrays("dtr_", d_trace_steps))
     if trace_g:
         out.update(rec_g.arrays("gtr_"))
         out["g_paths_flat"], out["g_paths_ptr"] = pflat, pptr
@@ -301,6 +304,10 @@ def random_graph(n, m, seed):
 
 
 def main():
+    global REF
+    if len(sys.argv) != 2:
+        sys.exit("usage: make_golden.py <reference checkout>")
+    REF = os.path.abspath(sys.argv[1])
     gg_mod, ref_utils = import_reference()
     # (1) the only golden vector in the reference: graph_gan.py:276-277
     import config as ref_config
@@ -340,10 +347,17 @@ def main():
     ids = np.asarray([int(l.split()[0]) for l in lines], np.int32)
     q = np.asarray([[int(round(float(x) * 1e6)) for x in l.split()[1:]] for l in lines], np.int32)
     assert np.array_equal(q.astype(np.float64) / 1e6, pre[ids])
-    extra = {"test_neg_edges": np.asarray(test_neg, np.int32), "pretrain_ids": ids, "pretrain_q1e6": q,
+    # rows in id order; q + 2**23 fits 24 bits and is stored as its three little-endian byte planes, which
+    # compress ~20 % smaller than int32 (the fixture stays below 1 MB; tests/golden/loader.py unpacks them)
+    order = np.argsort(ids)
+    ids, u = ids[order], q[order].astype(np.int64) + (1 << 23)
+    assert u.min() >= 0 and u.max() < (1 << 24)
+    planes = np.stack([(u >> s) & 255 for s in (0, 8, 16)]).astype(np.uint8)
+    extra = {"test_neg_edges": np.asarray(test_neg, np.int32), "pretrain_ids": ids, "pretrain_q1e6_bytes": planes,
              "pretrain_fill_seed": np.int64(123)}
+    # the D-pass trace is cut to the 6002 steps test_t1_teacher_forced_steps replays; d_steps / d_sum_l keep its totals
     run_case(gg_mod, ref_utils, "cagrqc", [tuple(e) for e in train], [tuple(e) for e in test], d=50, seed=2024,
-             emb=(pre, pre.copy()), trace_g=False, keep_parent=False, extra=extra)
+             emb=(pre, pre.copy()), trace_g=False, keep_parent=False, extra=extra, d_trace_steps=6002)
 
 
 if __name__ == "__main__":

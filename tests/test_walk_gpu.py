@@ -97,7 +97,7 @@ def test_stream_replay_matches_reference(name, hub, cuda_device):
     assert np.array_equal(lb[:n_rows].cpu().numpy(), case.d_labels)
     cnt = out.counters_host()
     assert cnt["stream_used"] == int(case.d_draws)
-    assert cnt["steps"] == case.dtr_chosen.shape[0]
+    assert cnt["steps"] == int(case.d_steps)
     assert _bits_to_set(dg.d1_bits.cpu().numpy(), hg.indptr, hg.adj) == set(map(tuple, case.mutated.tolist()))
     # G pass continues on the same stream
     used = cnt["stream_used"]
@@ -399,3 +399,35 @@ def test_empty_and_degenerate_batches(cuda_device):
     # (c) update_ratio = 0 skips every root
     out = smp.run(emb, bias, trees, dg.raw_deg, True, seed=1, update_ratio=0.0)
     assert out.counters_host()["accepted"] == 0 and (out.status.cpu().numpy()[:out.n_walks] == S.SKIPPED).all()
+
+
+def test_bench_dump_outputs_are_reproducible(cuda_device, tmp_path):
+    """`bench.py --dump-outputs DIR`: the D rows of the last timed step, float64, the same from run to run with the
+    same arguments; --steps sets the number of timed steps; the oracle parity of that step is clean."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for k in range(2):
+        d = tmp_path / ("run%d" % k)
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "powerlaw_100k", "--roots", "512",
+                              "--steps", "3", "--warmup", "1", "--no-cpu-baseline", "--g-steps", "0", "--verify", "4",
+                              "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600, cwd=root)
+        assert out.returncode == 0, out.stderr[-2000:]
+        line = json.loads(out.stdout)
+        assert line["steps"] == 3 and line["parity"]["mismatches"] == 0 and line["parity"]["tree_mismatches"] == 0
+        names = sorted(p.name for p in d.iterdir())
+        assert names == ["center.npy", "label.npy", "n_rows.npy", "neighbor.npy", "row_index.npy"]
+        assert sum(p.stat().st_size for p in d.iterdir()) <= 64 << 20
+        a = {p.stem: np.load(p) for p in d.iterdir()}
+        assert all(v.dtype == np.float64 for v in a.values())
+        n = int(a["n_rows"][0])
+        assert n > 0 and np.array_equal(a["row_index"], np.arange(n))       # small enough to be dumped whole
+        assert a["center"].shape == a["neighbor"].shape == a["label"].shape == (n,)
+        assert 2 * int(a["label"].sum()) == n                                # one negative row per positive row
+        assert ((a["neighbor"] >= 0) & (a["neighbor"] < 100_000)).all()
+        dumps.append(a)
+    for name in dumps[0]:
+        assert np.array_equal(dumps[0][name], dumps[1][name]), name
